@@ -34,7 +34,7 @@ N_BATCHES = int(os.environ.get('BM_BENCH_BATCHES', '40'))    # resident dataset:
 #                                      (BM_BENCH_BATCHES: dry runs on the host simulation only -- `config.l2_policy` states the size)
 LR, MOMENTUM, L2 = 0.05, 0.5, 1e-5
 REFERENCE_BUDGET_S = float(os.environ.get('BM_BENCH_REFERENCE_SECONDS', '40'))   # --impl reference: timed + warm-up steps together
-FIT_MIN_STEPS = int(os.environ.get('BM_BENCH_FIT_STEPS', '2000'))   # e2e: fit() runs at least this many steps (50 epochs of 40 batches)
+DUMP_BYTES = 64 * 2 ** 20                                     # --dump-outputs: at most this much in all
 FLOP_PER_STEP = 2.0 * B * V * H * (2 * K_GIBBS + 3)      # SURVEY.md §8(d): (2k+3) GEMMs of 2BVH
 
 RBM_WORKLOADS = {
@@ -212,6 +212,18 @@ def recorded_traffic(kernel_key):
     return None
 
 
+def dump_outputs(arrays, out_dir):
+    """Writes each array as out_dir/<name>.npy.  Past DUMP_BYTES in all, every array keeps the same fraction of its rows, a fixed
+    seeded sample, so that the files of two builds of the project compare element for element."""
+    total = sum(a.nbytes for a in arrays.values())
+    keep = min(1.0, DUMP_BYTES / total)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0:
+            a = a[np.sort(np.random.RandomState(0).choice(len(a), int(len(a) * keep), replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def blas_threads():
     try:
         from threadpoolctl import threadpool_limits
@@ -285,6 +297,7 @@ def rbm_workload(name, ctx, rank, world, compute):
               cfg_extra={'global_batch': b * world, 'k': k},
               kernel='bm::tc_program_kernel<2>')
     wl['step'] = lambda i: eng.train_step_at((i % n_batches) * b, b, lr, MOMENTUM, k, seed, i)
+    wl['outputs'] = eng.get_params                      # the trained variables: what the caller of a training step reads back
 
     def e2e_factory(kind_of_feed):
         # 'native': what fit() feeds for this data (bytes for binary data); 'float32': the same rows as grey levels --
@@ -305,11 +318,14 @@ def rbm_workload(name, ctx, rank, world, compute):
     def fit_e2e(n_steps, before_close=None):
         """The call a user of the library makes: Model(**kwargs).fit(X) on a HOST float32 array -- engine construction, weight
         initialisation, packing + page-locking of the training set, the epochs (every step uploads its own batch and reads its
-        MSRE back) and the final save are all inside the timed region.  Returns (seconds, steps run, bytes up per step)."""
+        MSRE back) and the final save are all inside the timed region.  Exactly `n_steps` steps: whole epochs over the first
+        `nb` batches of the dataset, `nb` the largest divisor of n_steps that it holds.  Returns (seconds, steps run, bytes up
+        per step)."""
         import shutil
         import tempfile
         from boltzmann_machines.rbm import BernoulliRBM, GaussianRBM
-        epochs = max(1, -(-n_steps // n_batches))
+        nb = max(d for d in range(1, min(n_batches, n_steps) + 1) if n_steps % d == 0)
+        epochs = n_steps // nb
         tmp = tempfile.mkdtemp(prefix='bm_bench_fit_')
         kw = dict(n_visible=v, n_hidden=h, W_init=w_std, hb_init=0., n_gibbs_steps=k, learning_rate=lr, momentum=MOMENTUM,
                   max_epoch=epochs, batch_size=b, l2=L2, sample_v_states=False, sample_h_states=True,
@@ -338,7 +354,7 @@ def rbm_workload(name, ctx, rank, world, compute):
         _native.CudaRBM.pin, NativeModel._save_model = timed('pin', real_pin), timed('save', real_save)
         try:
             t0 = time.perf_counter()
-            model.fit(X)
+            model.fit(X[:nb * b])
             ctx.sync()
             dt = time.perf_counter() - t0
             fit_e2e.breakdown_ms = {'pack_and_pin_training_set': 1e3 * spent['pin'], 'model_saves': 1e3 * spent['save'],
@@ -356,7 +372,7 @@ def rbm_workload(name, ctx, rank, world, compute):
                 _native.Context._default[None] = old
             shutil.rmtree(tmp, ignore_errors=True)
         byte_valued = _native.as_bytes(X[:64]) is not None
-        return dt, epochs * n_batches, b * v * (1 if byte_valued else 2)
+        return dt, epochs * nb, b * v * (1 if byte_valued else 2)
     wl['fit_e2e'] = fit_e2e
 
     def quality():
@@ -404,6 +420,7 @@ def dbm_workload(name, ctx, rank, world, compute, ais_runs, ais_betas):
                       ais_runs * (v + H1 + H2) * 6 // 2 ** 20),
                   cfg_extra={'n_runs': ais_runs, 'n_betas': ais_betas}, kernel='bm::tc_program_kernel<2>', step=step)
         wl['e2e_step'] = step                       # the call a user makes returns the log-weights to the host: same path
+        wl['outputs'] = lambda: {'logw': last['logw']}
         wl['h2d'] = 0
         wl['d2h'] = 8 * ais_runs
 
@@ -439,7 +456,7 @@ def dbm_workload(name, ctx, rank, world, compute, ais_runs, ais_betas):
                         'metric read-back only); weights + activations of a step: {0} MB'.format(
                             (4 * pairs * 3 + 2 * b * sum(sizes) * 6) // 2 ** 20),
               cfg_extra={'global_batch': b * world, 'k': k, 'max_mf_updates': cfg['max_mf_updates']},
-              kernel='bm::tc_program_kernel<2>', step=step, e2e_step=e2e_step)
+              kernel='bm::tc_program_kernel<2>', step=step, e2e_step=e2e_step, outputs=eng.get_params)
     wl['h2d'] = b * v * 4 * world
     wl['d2h'] = 16 * world
     wl['quality'] = lambda: {key: float(val) for key, val in nmf.items()}
@@ -552,7 +569,11 @@ def main():
     ap.add_argument('--compute', default='bf16')
     ap.add_argument('--ais-runs', type=int, default=20000)
     ap.add_argument('--ais-betas', type=int, default=1000)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed as DIR/<name>.npy (at most 64 MB: a fixed sample of larger outputs)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs: the reference arm times a sample of each step, not the outputs of the timed path')
     if args.steps is None:
         args.steps = {'cfg2': 2000, 'cfg3': 500, 'cfg5': 300, 'cfg5-pcd': 200, 'cfg4': 300, 'cfg4-ais': 3}[args.config]
     if args.impl == 'reference':
@@ -621,6 +642,11 @@ def main():
     launches = ctx.launch_count() - l0
     ms = max_over_ranks(ms)
     value = args.steps * units * world / (ms * 1e-3)
+    if args.dump_outputs:
+        # read before the regions below train on; the other ranks wait, since the read may reach their weight rows
+        if rank == 0:
+            dump_outputs(wl['outputs'](), args.dump_outputs)
+        barrier()
 
     # ---- region 2: same steps with per-launch CUDA events on the tensor-core kernel ---------------------------------
     ctx.profile_tc(True)
@@ -665,17 +691,15 @@ def main():
         # the headline end-to-end number goes through the public API itself: Model(...).fit(X)
         e2e['e2e_epoch_call'] = e2e.pop('e2e')
         barrier()
-        # fit() pays one-time costs (engine construction, packing and page-locking the training set, the save: about 0.1 s for
-        # this 514 MB float32 set) that a K-step run does not amortise when K is a few dozen: the fit runs for at least
-        # FIT_MIN_STEPS steps (whole epochs) whatever K is, and states how many it ran
-        fit_target = max(args.steps, FIT_MIN_STEPS if args.config == 'cfg2' else args.steps)
+        # fit() runs exactly K steps; its one-time costs (engine construction, packing and page-locking the training set, the
+        # save: about 0.1 s for the 514 MB float32 set of 40 batches) weigh less the larger K is
         try:
-            fit_s, fit_steps, up = wl['fit_e2e'](min(fit_target, 2 * wl['n_batches']), barrier)          # (warm: library loaded, CUDA context up)
+            fit_s, fit_steps, up = wl['fit_e2e'](min(args.steps, 2 * wl['n_batches']), barrier)          # (warm: library loaded, CUDA context up)
             passes = []
             for _ in range(2):
                 barrier()
                 sampler.mark()
-                fit_s, fit_steps, up = wl['fit_e2e'](fit_target, barrier)
+                fit_s, fit_steps, up = wl['fit_e2e'](args.steps, barrier)
                 barrier()
                 sampler.unmark()
                 passes.append(max_over_ranks(fit_s))

@@ -157,3 +157,145 @@ def run_example(path, argv, n_train=640, n_test=128):
             else:
                 sys.modules[k] = v
     return g
+
+
+# ---- what a script does with the package, recorded and replayed ---------------------------------------------------------
+# the package names the examples import; a trace refers to them by name
+ENTRY_POINTS = {'BernoulliRBM': ('boltzmann_machines.rbm', 'BernoulliRBM'), 'logit_mean': ('boltzmann_machines.rbm', 'logit_mean'),
+                'DBM': ('boltzmann_machines', 'DBM')}
+
+
+def summary(v):
+    """what a call returned, as far as a trace keeps it: shape and dtype of arrays, through dicts, lists and tuples"""
+    if isinstance(v, np.ndarray):
+        return {'shape': list(v.shape), 'dtype': v.dtype.name}
+    if isinstance(v, dict):
+        return {k: summary(x) for k, x in sorted(v.items())}
+    if isinstance(v, (list, tuple)):
+        return [summary(x) for x in v]
+    return None
+
+
+class _Model(object):
+    """a model the package returned to the script: its method calls are recorded"""
+
+    def __init__(self, recorder, obj, index):
+        self._recorder, self._obj, self._index = recorder, obj, index
+
+    def __getattr__(self, name):
+        attr = getattr(self._obj, name)
+        if not callable(attr):
+            return attr
+        return lambda *a, **kw: self._recorder.call({'call': self._index}, name, attr, a, kw)
+
+
+class _Entry(object):
+    """an entry point of the package as the script imports it: calling it, or a class method of it, is recorded"""
+
+    def __init__(self, recorder, name, real):
+        self._recorder, self._name, self._real = recorder, name, real
+
+    def __call__(self, *a, **kw):
+        return self._recorder.call({'entry': self._name}, '__call__', self._real, a, kw)
+
+    def __getattr__(self, attr):
+        real = getattr(self._real, attr)
+        return lambda *a, **kw: self._recorder.call({'entry': self._name}, attr, real, a, kw)
+
+
+def _unwrap(v):
+    if isinstance(v, _Model):
+        return v._obj
+    if isinstance(v, (list, tuple)):
+        return type(v)(_unwrap(x) for x in v)
+    if isinstance(v, dict):
+        return {k: _unwrap(x) for k, x in v.items()}
+    return v
+
+
+class Recorder(object):
+    """While active, the entry points of ENTRY_POINTS are wrappers that log every call into the package: the target (entry
+    point, or the model an earlier call returned), the method, the arguments and a summary of the result.  Arguments that are
+    results of earlier calls are referenced by call index, other arrays are kept in `arrays`, and paths are written relative to
+    `workdir`."""
+
+    def __init__(self, workdir):
+        self.workdir, self.calls, self.arrays, self._results, self._saved = workdir, [], {}, [], []
+
+    def __enter__(self):
+        import importlib
+        for name, (mod, attr) in ENTRY_POINTS.items():
+            m = importlib.import_module(mod)
+            self._saved.append((m, attr, getattr(m, attr)))
+            setattr(m, attr, _Entry(self, name, getattr(m, attr)))
+        return self
+
+    def __exit__(self, *exc):
+        for m, attr, real in self._saved:
+            setattr(m, attr, real)
+
+    def _encode(self, v):
+        if isinstance(v, _Model):
+            return {'call': v._index}
+        if isinstance(v, np.ndarray):
+            for i, r in enumerate(self._results):
+                if isinstance(r, np.ndarray) and (r is v or (r.shape == v.shape and r.dtype == v.dtype and np.array_equal(r, v))):
+                    return {'call': i}
+            for key, a in self.arrays.items():
+                if a.shape == v.shape and a.dtype == v.dtype and np.array_equal(a, v):
+                    return {'array': key}
+            key = 'a{0}'.format(len(self.arrays))
+            self.arrays[key] = v.copy()
+            return {'array': key}
+        if isinstance(v, (list, tuple)):
+            return {type(v).__name__: [self._encode(x) for x in v]}
+        if isinstance(v, dict):
+            return {'dict': {k: self._encode(x) for k, x in v.items()}}
+        if isinstance(v, str):
+            return v.replace(self.workdir, '{workdir}')
+        if isinstance(v, np.generic):
+            return v.item()
+        if v is None or isinstance(v, (bool, int, float)):
+            return v
+        raise TypeError('a trace cannot hold an argument of type {0}'.format(type(v)))
+
+    def call(self, target, method, fn, args, kwargs):
+        rec = {'target': target, 'method': method, 'args': [self._encode(a) for a in args],
+               'kwargs': {k: self._encode(v) for k, v in sorted(kwargs.items())}}
+        out = fn(*_unwrap(args), **_unwrap(kwargs))
+        rec['returned'] = summary(out)
+        self.calls.append(rec)
+        self._results.append(out)
+        if type(out).__module__.startswith('boltzmann_machines'):
+            return _Model(self, out, len(self.calls) - 1)
+        return out
+
+
+def replay(calls, arrays, workdir):
+    """Makes the calls of a trace on the package, in order, and checks that each returns what it returned when recorded (shapes
+    and dtypes of its arrays).  Returns every call's result."""
+    import importlib
+    results = []
+
+    def decode(v):
+        if isinstance(v, str):
+            return v.replace('{workdir}', workdir)
+        if not isinstance(v, dict):
+            return v
+        (tag, x), = v.items()
+        if tag == 'call':
+            return results[x]
+        if tag == 'array':
+            return arrays[x]
+        if tag == 'dict':
+            return {k: decode(y) for k, y in x.items()}
+        return {'list': list, 'tuple': tuple}[tag](decode(y) for y in x)
+
+    for c in calls:
+        t = c['target']
+        obj = getattr(importlib.import_module(ENTRY_POINTS[t['entry']][0]), ENTRY_POINTS[t['entry']][1]) if 'entry' in t else results[t['call']]
+        fn = obj if c['method'] == '__call__' else getattr(obj, c['method'])
+        out = fn(*[decode(a) for a in c['args']], **{k: decode(v) for k, v in c['kwargs'].items()})
+        assert summary(out) == c['returned'], (len(results), c['method'], summary(out), c['returned'])
+        results.append(out)
+    return results

@@ -1,17 +1,25 @@
-"""The reference's own example scripts run unchanged against this package (north_star; SURVEY.md section 8 f.1): read from the
-reference checkout, Python-2 syntax rewritten in memory, Keras / the MNIST loader replaced by stand-ins (tests/example_runner.py).
-Here on the CPU with the oracle engines (the host logic is the same whichever engine computes); skipped where the reference
-checkout does not exist (the GPU box)."""
+"""The reference's own example scripts against this package (north_star; SURVEY.md section 8 f.1).  The scripts are the original
+project's source and stay out of this repository: tests/golden/make_example_traces.py ran them UNCHANGED (Python-2 syntax rewritten
+in memory, Keras / the MNIST loader replaced by stand-ins: tests/example_runner.py), twice each -- training, then the rerun that
+takes the load_model branches -- and recorded every call they made into the package.  These tests make the same calls, on the
+CPU with the oracle engines (the host logic is the same whichever engine computes), and check what the scripts went on to use."""
 import json
 import os
 
 import numpy as np
-import pytest
 
-from example_runner import run_example, translate
+from example_runner import replay, translate
 
-EXAMPLES = '/root/reference/examples'
-needs_reference = pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason='the reference checkout is not on this machine')
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+
+
+def replay_example(name, workdir):
+    with open(os.path.join(GOLDEN, 'example_{0}_trace.json'.format(name))) as fh:
+        calls = json.load(fh)['calls']
+    with np.load(os.path.join(GOLDEN, 'example_{0}_trace.npz'.format(name))) as z:
+        arrays = {k: z[k] for k in z.files}
+    results = replay(calls, arrays, str(workdir))
+    return {c['method']: [r for d, r in zip(calls, results) if d['method'] == c['method']] for c in calls}
 
 
 def test_translate_handles_the_two_python2_constructs_of_the_examples():
@@ -21,38 +29,23 @@ def test_translate_handles_the_two_python2_constructs_of_the_examples():
     assert g['f']((1, 2), 3, (4, 5)) == 6
 
 
-@needs_reference
-def test_rbm_mnist_example_runs_unchanged(oracle_engines, tmp_path, capsys):
-    model = str(tmp_path / 'rbm') + '/'
-    args = ['--n-train', '512', '--n-val', '128', '--n-hidden', '48', '--epochs', '2', '--batch-size', '64',
-            '--model-dirpath', model, '--mlp-save-prefix', str(tmp_path) + '/rbm_', '--mlp-epochs', '1']
-    run_example(os.path.join(EXAMPLES, 'rbm_mnist.py'), args)
-    out = capsys.readouterr().out
-    assert 'Training model' in out and 'Test accuracy' in out
-    params = json.load(open(os.path.join(model, 'params.json')))
+def test_rbm_mnist_example_runs_unchanged(oracle_engines, tmp_path):
+    got = replay_example('rbm_mnist', tmp_path)
+    params = json.load(open(str(tmp_path / 'rbm' / 'params.json')))
     assert params['n_hidden'] == 48 and params['epoch_'] == 2
-    W = np.load(str(tmp_path) + '/rbm_W_finetuned.npy')             # what the script hands to Keras: the trained RBM weights
-    assert W.shape == (784, 48) and np.abs(W).max() > 0.011
-    # a second run finds the model directory and takes the script's load_model branch
-    run_example(os.path.join(EXAMPLES, 'rbm_mnist.py'), args)
-    assert 'Loading model' in capsys.readouterr().out
+    trained, loaded = got['get_tf_params']                # what the script hands to Keras: the trained RBM weights
+    assert trained['W'].shape == (784, 48) and np.abs(trained['W']).max() > 0.011
+    # the rerun finds the model directory and takes the script's load_model branch
+    assert len(got['load_model']) == 1 and all(np.array_equal(trained[k], loaded[k]) for k in trained)
 
 
-@needs_reference
-def test_dbm_mnist_example_runs_unchanged(oracle_engines, tmp_path, capsys):
-    d = str(tmp_path)
-    args = ['--n-train', '256', '--n-val', '64', '--n-hiddens', '32', '24', '--epochs', '1', '1', '2', '--batch-size', '32', '32', '32',
-            '--increase-n-gibbs-steps-every', '1', '--n-particles', '32', '--max-mf-updates', '5',
-            '--rbm1-dirpath', d + '/rbm1/', '--rbm2-dirpath', d + '/rbm2/', '--dbm-dirpath', d + '/dbm/',
-            '--mlp-save-prefix', d + '/dbm_', '--mlp-epochs', '1']
-    run_example(os.path.join(EXAMPLES, 'dbm_mnist.py'), args)
-    out = capsys.readouterr().out
-    assert 'Training RBM #1' in out and 'Training RBM #2' in out and 'Training DBM' in out and 'Test accuracy' in out
-    params = json.load(open(d + '/dbm/params.json'))
+def test_dbm_mnist_example_runs_unchanged(oracle_engines, tmp_path):
+    got = replay_example('dbm_mnist', tmp_path)
+    assert len(got['fit']) == 3 and len(got['transform']) == 2          # RBM #1, RBM #2 (each feeding the next), the DBM
+    params = json.load(open(str(tmp_path / 'dbm' / 'params.json')))
     assert params['n_hiddens_'] == [32, 24] and params['epoch_'] == 2
-    W1, W2 = np.load(d + '/dbm_W1_finetuned.npy'), np.load(d + '/dbm_W2_finetuned.npy')
-    assert W1.shape == (784, 32) and W2.shape == (32, 24)
-    # second run: every model is loaded from disk, `dbm.load_rbms(rbms)` included (dbm_mnist.py:133-134)
-    run_example(os.path.join(EXAMPLES, 'dbm_mnist.py'), args)
-    out = capsys.readouterr().out
-    assert 'Loading RBM #1' in out and 'Loading DBM' in out
+    trained, loaded = got['get_tf_params']
+    assert trained['W'].shape == (784, 32) and trained['W_1'].shape == (32, 24)
+    # the rerun loads every model from disk, `dbm.load_rbms(rbms)` included (dbm_mnist.py:133-134)
+    assert len(got['load_model']) == 3 and len(got['load_rbms']) == 1
+    assert all(np.array_equal(trained[k], loaded[k]) for k in trained)
